@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rasterizer forward+backward frames/s at BASELINE.json's headline configuration.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[1] -- ~100k mesh-bound splats, 1920x1080, SH degree 3, fused
@@ -27,6 +27,10 @@ camera, "scaling": "weak").
            is a PROXY for the absent upstream CUDA rasterizer (same kernels underneath, minus the fusion and the
            culling), not a measurement of it.
   roofline / cpu_baseline : see DESIGN.md "Measurement".
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last of them computed -- the image, the radii and
+the gradients of the raw splat parameters and of the posed mesh vertices -- as DIR/<name>.npy (float32).  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -48,6 +52,9 @@ P_SPLATS = 100_000
 WIDTH, HEIGHT = 1920, 1080
 SH_DEGREE = 3
 N_CAMERAS = 16  # distinct orbit views cycled through
+DUMP_BYTES = 63_900_000  # --dump-outputs: all arrays together, room left for the .npy headers within 64 MB
+# names of the gradients of MeshBoundGaussians.parameters(), in its order
+PARAM_NAMES = ("xyz", "rotation", "scaling", "opacity", "features_dc", "features_rest")
 METRIC = "rasterizer fwd+bwd frames/sec @100k splats 1080p"
 WORKLOAD = "avatar-100k-splats-1920x1080-sh3-fused-binding-fwd+bwd (BASELINE configs[1], synthetic media/306 stand-in)"
 
@@ -93,7 +100,13 @@ def parse():
     ap.add_argument("--width", type=int, default=None)
     ap.add_argument("--height", type=int, default=None)
     ap.add_argument("--cameras", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (native arm)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native path")
     global P_SPLATS, WIDTH, HEIGHT, N_CAMERAS, WORKLOAD
     if a.splats or a.width or a.height or a.cameras:
         P_SPLATS = a.splats or P_SPLATS
@@ -262,8 +275,7 @@ def run_reference(args, rank, world):
     params = syn.avatar_splats(P_SPLATS, n_faces=faces.shape[0], seed=0, sh_degree=SH_DEGREE)
     cams = make_cameras(N_CAMERAS)
     cores = host_cpus()
-    # bounded sample: one frame per step, steps capped so the whole run stays within ~2 minutes
-    steps = max(1, min(args.steps, 12))
+    steps = args.steps   # one frame per step
     warm = max(1, min(args.warmup, 2))
     cpu_frames(params, verts, faces, cams, warm)
     t, _ = cpu_frames(params, verts, faces, cams, steps)
@@ -514,9 +526,12 @@ def main():
             fr.capture()
         return pair
 
+    last_eager = {}
+
     def step_resident(i):
         if not frames:
-            return step_eager(i)
+            last_eager["out"] = step_eager(i)
+            return
         fr = frames[i % len(frames)]
         fr.set_inputs(camera=cam_blocks_dev[i % len(cam_blocks_dev)], verts=posed[i % len(posed)].detach())
         fr.run()
@@ -551,6 +566,15 @@ def main():
     # the headline number: nothing but the K steps (+ the drained K-th reduction) inside the event pairs
     ms_total, _, clk, wall_timed, _, _ = timed_pass(step_resident, False, tail=drain if deferred else None)
     overflow_steps = any(fr.overflowed(wait=True) for fr in frames)
+    if args.dump_outputs and rank == 0:
+        if frames:
+            fr = frames[(K - 1) % len(frames)]
+            image, radii, grad_verts = fr.image, fr.radii, fr.verts.grad
+        else:
+            out = last_eager["out"]
+            image, radii, grad_verts = out["render"], out["radii"], posed[(K - 1) % len(posed)].grad
+        dump_outputs(args.dump_outputs, {"image": image, "radii": radii, "grad_verts": grad_verts,
+                                         **{"grad_" + n: p.grad for n, p in zip(PARAM_NAMES, pc.parameters())}})
 
     # ---- warm-L2 variant (no flush), whole-loop events: what a training loop actually sees -------------------
     barrier()
@@ -802,6 +826,28 @@ def main():
         line.update(cpu_and_parity(params, verts, faces, cams_host, pc, posed, cams_dev, bg, gout, dev))
     print(json.dumps(line), flush=True)
     finish(world, dev)
+
+
+def dump_outputs(directory, tensors):
+    """Writes each tensor as <directory>/<name>.npy in float32 (float64 stays float64).  When together they would exceed
+    DUMP_BYTES, every one is flattened and keeps the same share of its elements, chosen with a fixed seed and kept in
+    their original order, so that two runs of the same configuration write the same elements."""
+    import numpy as np
+
+    host = {}
+    for name, t in tensors.items():
+        if t is None:
+            raise RuntimeError(f"--dump-outputs: the timed step produced no {name}")
+        a = t.detach().cpu().numpy()
+        host[name] = a.astype(np.float64 if a.dtype == np.float64 else np.float32, copy=False)
+    total = sum(a.nbytes for a in host.values())
+    share = min(1.0, DUMP_BYTES / total) if total else 1.0
+    os.makedirs(directory, exist_ok=True)
+    for name, a in host.items():
+        if share < 1.0:
+            n = max(1, int(a.size * share))
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, n, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def finish(world, dev):

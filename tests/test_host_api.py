@@ -31,7 +31,12 @@ def test_library_exports_every_declared_symbol():
     assert lib.gab200_abi_version() == N.ABI_VERSION == 3
     assert b"invalid argument" in lib.gab200_status_string(-1)
     assert b"sm_100" in lib.gab200_status_string(-4)
-    assert lib.gab200_launch_count() == 0
+    # loading the library and the calls above launch nothing; counted in a fresh process, since the GPU tests that
+    # share this one have launched kernels
+    code = ("from gaussianavatars_b200 import _native as N; lib = N.lib(); lib.gab200_abi_version(); "
+            "lib.gab200_status_string(-1); lib.gab200_status_string(-4); print(lib.gab200_launch_count())")
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=ROOT)
+    assert out.returncode == 0 and out.stdout.split()[-1:] == ["0"], (out.stdout, out.stderr)
 
 
 def test_ctypes_structs_match_the_c_layout(tmp_path):

@@ -1,6 +1,7 @@
 """CPU: the splat PLY format (gaussianavatars_b200/io.py) against the reference's writer/reader
-(scene/gaussian_model.py:234-332) and, when /root/reference is mounted, against the demo avatar it ships."""
+(scene/gaussian_model.py:234-332) and against samples of the demo avatar it ships (tests/golden/make_golden_demo.py)."""
 import hashlib
+import json
 import os
 
 import numpy as np
@@ -9,7 +10,9 @@ import torch
 
 from gaussianavatars_b200 import io as gio
 
-DEMO = "/root/reference/media/306/point_cloud.ply"
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
+FACTS = json.load(open(os.path.join(GOLDEN, "reference_facts.json")))
+DEMO = os.path.join(GOLDEN, "demo_point_cloud_sample.ply")   # media/306/point_cloud.ply: a sample of its records
 # sha256 of the 1555-byte header of media/306/point_cloud.ply (89,021 vertices, 63 float properties incl. binding_0),
 # recorded from the real file: pins `ply_header` to plyfile's output without shipping the asset
 DEMO_HEADER_SHA256 = "4f7c89da20e1671bf40dae12e75a21aeabe7c91ec9cf9ec980479f234363cbda"
@@ -122,13 +125,19 @@ def test_loaded_parameters_drive_the_bound_model():
     assert torch.equal(a.binding, b.binding)
 
 
-@pytest.mark.skipif(not os.path.exists(DEMO), reason="/root/reference is not mounted here")
 def test_demo_avatar_of_the_reference_round_trips_byte_for_byte(tmp_path):
+    facts = FACTS["point_cloud"]
+    raw = open(DEMO, "rb").read()
+    hdr = raw[:raw.index(b"end_header\n") + len(b"end_header\n")]
+    # the sample sits under the demo file's own header, vertex count aside
+    full = hdr.replace(b"element vertex %d\n" % facts["vertices"], b"element vertex %d\n" % facts["source_vertices"])
+    assert facts["source_vertices"] == 89021 and hashlib.sha256(full).hexdigest() == DEMO_HEADER_SHA256
     d = gio.load_ply(DEMO)
     P = d["_xyz"].shape[0]
-    assert P == 89021 and d["_features_rest"].shape == (P, 15, 3) and d["binding"].dtype == torch.int32
-    assert int(d["binding"].min()) == 0 and int(d["binding"].max()) == 10143       # SURVEY.md 8(d) config 2
-    assert abs(float(torch.sigmoid(d["_opacity"]).mean()) - 0.458) < 1e-3
+    assert P == facts["vertices"] and d["_features_rest"].shape == (P, 15, 3) and d["binding"].dtype == torch.int32
+    assert (facts["source_binding_min"], facts["source_binding_max"]) == (0, 10143)   # SURVEY.md 8(d) config 2
+    assert int(d["binding"].min()) == facts["binding_min"] and int(d["binding"].max()) == facts["binding_max"]
+    assert abs(float(torch.sigmoid(d["_opacity"].double()).mean()) - facts["opacity_sigmoid_mean"]) < 1e-9
     out = tmp_path / "again.ply"
     gio.save_ply(str(out), d)
     h1, h2 = hashlib.sha256(), hashlib.sha256()
@@ -140,7 +149,7 @@ def test_demo_avatar_of_the_reference_round_trips_byte_for_byte(tmp_path):
 # ------------------------------------------------------------------------------------------------------------
 # flame_param.npz
 # ------------------------------------------------------------------------------------------------------------
-DEMO_NPZ = "/root/reference/media/306/flame_param.npz"
+DEMO_NPZ = os.path.join(GOLDEN, "demo_flame_param_sample.npz")   # media/306/flame_param.npz: frames and vertices cut
 
 
 def _fake_flame(T, V=37, seed=0):
@@ -174,15 +183,17 @@ def test_flame_param_round_trip_and_motion_override(tmp_path, mmap):
         assert torch.equal(mixed[k], mo[k]) and mixed[k].shape[0] == 9
 
 
-@pytest.mark.skipif(not os.path.exists(DEMO_NPZ), reason="/root/reference is not mounted here")
 def test_flame_param_of_the_demo_avatar(tmp_path):
     """media/306/flame_param.npz: mapped in place == np.load, and re-saved member by member byte-identical (the .npy
     payloads; zip timestamps differ between any two np.savez calls)."""
     import zipfile
 
+    facts = FACTS["flame_param"]
+    T, V = facts["frames"], facts["vertices"]
     fp = gio.load_flame_param(DEMO_NPZ)
-    assert fp["expr"].shape == (1119, 100) and fp["static_offset"].shape == (1, 5143, 3) and fp["shape"].shape == (300,)
-    assert fp["dynamic_offset"].shape == (1119, 5143, 3) and fp["eyes_pose"].shape == (1119, 6)
+    assert {k: list(v.shape) for k, v in fp.items()} == facts["shapes"]
+    assert fp["expr"].shape == (T, 100) and fp["static_offset"].shape == (1, V, 3) and fp["shape"].shape == (300,)
+    assert fp["dynamic_offset"].shape == (T, V, 3) and fp["eyes_pose"].shape == (T, 6)
     z = np.load(DEMO_NPZ)
     small = [k for k in z.files if k != "dynamic_offset"]
     for k in small:
