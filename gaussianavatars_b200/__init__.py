@@ -10,7 +10,9 @@ from .renderer import render, render_bound
 from .training import photometric_loss, Adam, binding_regularizers
 from .io import load_ply, save_ply, load_flame_param, save_flame_param
 from .densify import densify_and_prune, densify_arrays
+from .flame import FusedFlameHead
 
 __all__ = ["GaussianRasterizationSettings", "GaussianRasterizer", "rasterize_gaussians", "rasterize_bound",
            "bind_activate", "set_exact_binning", "face_frame", "l1_loss_u8", "render", "render_bound",
-           "photometric_loss", "Adam", "binding_regularizers", "load_ply", "save_ply", "load_flame_param", "save_flame_param", "densify_and_prune", "densify_arrays"]
+           "photometric_loss", "Adam", "binding_regularizers", "load_ply", "save_ply", "load_flame_param", "save_flame_param", "densify_and_prune", "densify_arrays",
+           "FusedFlameHead"]

@@ -126,6 +126,22 @@ class RegularizeArgs(C.Structure):
     ]
 
 
+class FlameArgs(C.Structure):
+    """Mirror of gab200_flame_args."""
+    _fields_ = [
+        ("abi_version", C.c_uint32), ("V", C.c_int32), ("n_shape", C.c_int32), ("n_expr", C.c_int32),
+        ("J", C.c_int32), ("T", C.c_int32),
+        ("v_template", C.c_void_p), ("shapedirs", C.c_void_p), ("posedirs", C.c_void_p), ("J_regressor", C.c_void_p),
+        ("lbs_weights", C.c_void_p), ("parents", C.c_void_p), ("J_template", C.c_void_p), ("J_shapedirs", C.c_void_p),
+        ("row", C.c_void_p), ("shape", C.c_void_p), ("expr", C.c_void_p), ("rotation", C.c_void_p), ("neck", C.c_void_p),
+        ("jaw", C.c_void_p), ("eyes", C.c_void_p), ("translation", C.c_void_p), ("static_offset", C.c_void_p),
+        ("verts", C.c_void_p), ("verts_cano", C.c_void_p), ("workspace", C.c_void_p),
+        ("grad_shape", C.c_void_p), ("grad_expr", C.c_void_p), ("grad_rotation", C.c_void_p), ("grad_neck", C.c_void_p),
+        ("grad_jaw", C.c_void_p), ("grad_eyes", C.c_void_p), ("grad_translation", C.c_void_p),
+        ("grad_static_offset", C.c_void_p),
+    ]
+
+
 ADAM_MAX_SEGMENTS = 8
 PHOTOMETRIC_SCRATCH_HEAD = 4
 
@@ -134,7 +150,8 @@ EXPORTED_SYMBOLS = ("gab200_forward", "gab200_backward", "gab200_mark_visible", 
                     "gab200_stage_timing_enable", "gab200_stage_times", "gab200_face_frame_forward",
                     "gab200_face_frame_backward", "gab200_host_times", "gab200_l1_loss_u8", "gab200_l1_loss_u8_backward",
                     "gab200_photometric_loss", "gab200_adam_step", "gab200_tune", "gab200_counters_ok",
-                    "gab200_regularize_forward", "gab200_regularize_backward", "gab200_nvls_allreduce", "gab200_densify_scratch_bytes", "gab200_densify_plan", "gab200_densify_apply")
+                    "gab200_regularize_forward", "gab200_regularize_backward", "gab200_nvls_allreduce", "gab200_densify_scratch_bytes", "gab200_densify_plan", "gab200_densify_apply",
+                    "gab200_flame_workspace_bytes", "gab200_flame_forward", "gab200_flame_backward")
 
 _lib = None
 _lock = threading.Lock()
@@ -190,6 +207,12 @@ def lib():
         L.gab200_densify_plan.argtypes = [C.POINTER(DensifyArgs), C.c_void_p]
         L.gab200_densify_apply.restype = C.c_int32
         L.gab200_densify_apply.argtypes = [C.POINTER(DensifyArgs), C.POINTER(DensifyOut), C.c_void_p]
+        L.gab200_flame_workspace_bytes.restype = C.c_size_t
+        L.gab200_flame_workspace_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32]
+        L.gab200_flame_forward.restype = C.c_int32
+        L.gab200_flame_forward.argtypes = [C.POINTER(FlameArgs), C.c_void_p]
+        L.gab200_flame_backward.restype = C.c_int32
+        L.gab200_flame_backward.argtypes = [C.POINTER(FlameArgs), C.c_void_p, C.c_void_p]
         L.gab200_counters_ok.restype = C.c_int32
         L.gab200_counters_ok.argtypes = [C.c_void_p, C.c_uint32]
         L.gab200_l1_loss_u8.restype = C.c_int32

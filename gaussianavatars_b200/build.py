@@ -30,6 +30,7 @@ SOURCES = {
     "nvls.cu": [],
     "blend.cu": [],
     "face_frame.cu": [],
+    "flame.cu": [],
     "loss.cu": [],
     "optim.cu": [],
 }

@@ -731,6 +731,36 @@ int32_t gab200_face_frame_backward(int32_t F, int32_t V, const float* verts, con
   return cudaPeekAtLastError() == cudaSuccess ? GAB200_OK : GAB200_ERR_CUDA;
 }
 
+static bool flame_args_ok(const gab200_flame_args* a) {
+  if (a == nullptr || a->abi_version != GAB200_ABI_VERSION) return false;
+  if (a->J != 5 || a->V <= 0 || a->n_shape < 0 || a->n_expr < 0 || a->T <= 0) return false;
+  if (!a->v_template || !a->shapedirs || !a->posedirs || !a->J_regressor || !a->lbs_weights || !a->parents ||
+      !a->J_template || !a->J_shapedirs)
+    return false;
+  if ((a->n_expr > 0 && !a->expr) || !a->rotation || !a->neck || !a->jaw || !a->eyes || !a->translation) return false;
+  if (!a->verts || !a->workspace || ((uintptr_t)a->workspace & 255) != 0) return false;
+  return true;
+}
+
+size_t gab200_flame_workspace_bytes(int32_t V, int32_t n_shape, int32_t n_expr) {
+  if (V < 0 || n_shape < 0 || n_expr < 0) return 0;
+  return flame_workspace_bytes(V, n_shape + n_expr);
+}
+
+int32_t gab200_flame_forward(const gab200_flame_args* a, void* stream_) {
+  if (!flame_args_ok(a)) return GAB200_ERR_INVALID_ARGUMENT;
+  if (check_arch() < 0) return GAB200_ERR_ARCH;
+  launch_flame_forward(*a, (cudaStream_t)stream_);
+  return cudaPeekAtLastError() == cudaSuccess ? GAB200_OK : GAB200_ERR_CUDA;
+}
+
+int32_t gab200_flame_backward(const gab200_flame_args* a, const float* dL_dverts, void* stream_) {
+  if (!flame_args_ok(a) || dL_dverts == nullptr) return GAB200_ERR_INVALID_ARGUMENT;
+  if (check_arch() < 0) return GAB200_ERR_ARCH;
+  launch_flame_backward(*a, dL_dverts, (cudaStream_t)stream_);
+  return cudaPeekAtLastError() == cudaSuccess ? GAB200_OK : GAB200_ERR_CUDA;
+}
+
 int32_t gab200_l1_loss_u8(int64_t n, const float* img, const uint8_t* gt, float* grad, float* loss, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   if (n < 0 || !loss || (n > 0 && (!img || !gt))) return GAB200_ERR_INVALID_ARGUMENT;

@@ -164,6 +164,11 @@ void launch_face_frame_forward(int F, const float* verts, const int32_t* faces, 
 void launch_face_frame_backward(int F, const float* verts, const int32_t* faces, const float* g_fc, const float* g_fR,
                                 const float* g_fs, float* g_verts, cudaStream_t stream);
 
+// flame.cu
+size_t flame_workspace_bytes(int V, int NB);
+void launch_flame_forward(const gab200_flame_args& a, cudaStream_t stream);
+void launch_flame_backward(const gab200_flame_args& a, const float* g_verts, cudaStream_t stream);
+
 // loss.cu
 void launch_l1_loss_u8(int64_t n, const float* img, const uint8_t* gt, const float* upstream, float* grad, float* loss,
                        cudaStream_t stream);

@@ -88,7 +88,8 @@ class GraphedFrame:
     def __init__(self, pc, width: int, height: int, fovx: float, fovy: float, bg: torch.Tensor, loss: str = "l1_u8",
                  lambda_dssim: float = 0.2, host_inputs: bool = False, capacity: Optional[int] = None,
                  headroom: float = 1.25, after_backward=None, warm_cameras=None, regularizers: Optional[dict] = None,
-                 before_backward=None, side_work=None, side_work_at: str = "start"):
+                 before_backward=None, side_work=None, side_work_at: str = "start", flame=None, flame_param=None,
+                 warm_timesteps=None):
         """loss: "l1_u8" (L1 vs a uint8 ground truth), "photometric" ((1-l) L1 + l (1-SSIM) vs a uint8 ground truth) or
         "dL_dimage" (the caller supplies dL/dimage in `self.dL_dimage`).
         host_inputs: the frame owns pinned STAGING tensors (`cam_stage` (35,) float32, `gt_stage` (3,H,W) uint8) that a
@@ -108,7 +109,13 @@ class GraphedFrame:
         (dist.SymmetricGradBuffer.reduce of the other frame of an alternating pair), which then costs no step time.
         warm_cameras: camera blocks (35,) rendered eagerly before the capture to size the instance capacity.
         regularizers: keyword arguments of `binding_regularizers` (threshold_xyz, lambda_scale, ...; {} = the
-        reference's defaults): the position / scale terms of train.py:134-146 are added to the loss inside the graph."""
+        reference's defaults): the position / scale terms of train.py:134-146 are added to the loss inside the graph.
+        flame / flame_param: a FusedFlameHead and its parameters (io.load_flame_param's layout).  The graph then starts
+        from a device timestep (`set_inputs(timestep=t)`) instead of posed vertices: FLAME forward -> face frame -> ...
+        -> backward -> FLAME backward, and after each replay the `.grad` of every flame_param tensor that requires grad
+        is the graph's static (T,k) gradient (one non-zero row).  warm_timesteps: the timesteps of the eager frames
+        that size the instance capacity.  FLAME gradients are not all-reduced, so this mode refuses a process group of
+        more than one rank."""
         if loss not in ("l1_u8", "photometric", "dL_dimage"):
             raise ValueError("loss must be 'l1_u8', 'photometric' or 'dL_dimage'")
         self.pc, self.W, self.H, self.fovx, self.fovy = pc, int(width), int(height), float(fovx), float(fovy)
@@ -126,7 +133,20 @@ class GraphedFrame:
         self.bg = bg.to(dev).float().contiguous()
         self.cam = torch.zeros(35, dtype=torch.float32, device=dev)
         self.camera = _GraphCamera(self.W, self.H, self.fovx, self.fovy, self.cam)
-        self.verts = pc.verts_rest.detach().clone().contiguous().requires_grad_(True)
+        if (flame is None) != (flame_param is None):
+            raise ValueError("flame and flame_param go together")
+        if flame is not None and torch.distributed.is_available() and torch.distributed.is_initialized() \
+                and torch.distributed.get_world_size() > 1:
+            raise RuntimeError("GraphedFrame(flame=...) does not all-reduce the FLAME-parameter gradients: with "
+                               f"{torch.distributed.get_world_size()} ranks the replicas would diverge")
+        self.flame, self.flame_param = flame, flame_param
+        if flame is None:
+            self.verts = pc.verts_rest.detach().clone().contiguous().requires_grad_(True)
+            self.timestep = None
+        else:   # posed by the graph itself: `verts` is the FLAME output of the last replay
+            self.verts = None
+            self.timestep = torch.zeros(1, dtype=torch.int32, device=dev)
+        self._warm_t = list(warm_timesteps) if warm_timesteps is not None else None
         self.gt = torch.zeros((3, self.H, self.W), dtype=torch.uint8, device=dev) if loss != "dL_dimage" else None
         self.dL_dimage = torch.zeros((3, self.H, self.W), dtype=torch.float32, device=dev) if loss == "dL_dimage" else None
         self.cam_host = torch.zeros(35, dtype=torch.float32).pin_memory() if host_inputs else None  # staging
@@ -148,8 +168,19 @@ class GraphedFrame:
         self._warm = list(warm_cameras) if warm_cameras is not None else None
 
     # ---- inputs ------------------------------------------------------------------------------------------------
-    def set_inputs(self, camera=None, verts=None, gt_u8=None, dL_dimage=None):
-        """Copies new inputs into the static buffers (device tensors) / staging buffers (host_inputs)."""
+    def set_inputs(self, camera=None, verts=None, gt_u8=None, dL_dimage=None, timestep=None):
+        """Copies new inputs into the static buffers (device tensors) / staging buffers (host_inputs).  `timestep`
+        (an int or an int32 tensor) is the FLAME frame of a graph built with flame=; `verts` is the posed mesh of one
+        built without."""
+        if self.flame is not None and verts is not None:
+            raise ValueError("this GraphedFrame poses the mesh with FLAME: pass timestep=, not verts=")
+        if self.flame is None and timestep is not None:
+            raise ValueError("timestep= needs a GraphedFrame built with flame= and flame_param=")
+        if timestep is not None:
+            if isinstance(timestep, torch.Tensor):
+                self.timestep.copy_(timestep.reshape(1), non_blocking=True)
+            else:
+                self.timestep.fill_(int(timestep))
         if camera is not None:
             blk = camera if isinstance(camera, torch.Tensor) else camera_block(camera)
             if blk.device.type == "cpu" and self._uploads:
@@ -196,13 +227,17 @@ class GraphedFrame:
 
     # ---- the step body (run eagerly for warm-up, then captured) --------------------------------------------------
     def _params(self):
-        return list(self.pc.parameters())
+        ps = list(self.pc.parameters())
+        if self.flame_param is not None:
+            ps += [t for t in self.flame_param.values() if isinstance(t, torch.Tensor) and t.requires_grad]
+        return ps
 
     def _body(self):
         pc = self.pc
         for p in self._params():
             p.grad = None
-        self.verts.grad = None
+        if self.flame is None:
+            self.verts.grad = None
         other = self._prefetch_target
         forked = other is not None or self.side_work is not None
         if forked:   # forked branch: runs while this frame computes
@@ -215,6 +250,8 @@ class GraphedFrame:
                         other.gt.copy_(other.gt_stage, non_blocking=True)
                 if self.side_work is not None and self.side_work_at == "start":
                     self.side_work()
+        if self.flame is not None:
+            self.verts = self.flame.mesh_at(self.flame_param, self.timestep)
         pc.update_mesh_properties(self.verts)
         out = render(self.camera, pc, _Pipe, self.bg)
         img = out["render"]
@@ -256,6 +293,9 @@ class GraphedFrame:
         key = (self.device, self.W, self.H, self.pc._xyz.shape[0])
         n_max, lo, hi = 0, 0xFFFFFFFF, 0
         blocks = self._warm if self._warm else [self.cam.clone()]
+        steps = [None]
+        if self.flame is not None:
+            steps = self._warm_t if self._warm_t else [self.timestep.clone()]
         # eager frames on a side stream (torch's recipe for whole-step capture): nothing autograd creates here may be
         # tied to the legacy default stream
         cur = torch.cuda.current_stream(self.device)
@@ -263,8 +303,10 @@ class GraphedFrame:
         side.wait_stream(cur)
         with torch.cuda.stream(side):
             for rep in range(2):
-                for blk in blocks:
+                for blk, ts in [(b, t) for b in blocks for t in steps]:
                     self.cam.copy_(blk)
+                    if ts is not None:
+                        self.set_inputs(timestep=ts)
                     self._body()
                     info = hints.last or {}
                     n_max = max(n_max, int(info.get("num_rendered", 0)))
@@ -276,6 +318,8 @@ class GraphedFrame:
         # release what the eager frames left on the model / on this object (tensors with autograd history)
         self.pc.face_center = self.pc.face_orien_mat = self.pc.face_scaling = None
         self.image = self.radii = self.viewspace_points = self.loss = None
+        if self.flame is not None:
+            self.verts = None
         return n_max, ((lo, hi) if hi > lo else (0, 0))
 
     def capture(self, capacity: Optional[int] = None):

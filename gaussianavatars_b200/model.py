@@ -73,7 +73,16 @@ def quat_mul_wxyz(p: torch.Tensor, q: torch.Tensor) -> torch.Tensor:
 class MeshBoundGaussians:
     def __init__(self, params: Dict[str, torch.Tensor], sh_degree: int, verts: Optional[torch.Tensor] = None,
                  faces: Optional[torch.Tensor] = None, pose_fn: Optional[Callable] = None, device="cuda",
-                 requires_grad: bool = False):
+                 requires_grad: bool = False, flame=None, flame_param: Optional[Dict[str, torch.Tensor]] = None):
+        """flame / flame_param: a FusedFlameHead and its parameters (io.load_flame_param's layout): the mesh of
+        `select_mesh_by_timestep(t)` is then `flame.mesh_at(flame_param, t)`; `verts` / `faces` default to the
+        FLAME template and faces.  Otherwise the mesh is `pose_fn(verts, t)` (or `verts` itself)."""
+        if (flame is None) != (flame_param is None):
+            raise ValueError("flame and flame_param go together")
+        if flame is not None:
+            verts = flame.v_template if verts is None else verts
+            faces = flame.faces if faces is None else faces
+        self.flame, self.flame_param = flame, flame_param
         self.max_sh_degree = sh_degree
         self.active_sh_degree = sh_degree
         for k in ("_xyz", "_rotation", "_scaling", "_opacity", "_features_dc", "_features_rest"):
@@ -114,7 +123,10 @@ class MeshBoundGaussians:
 
     def select_mesh_by_timestep(self, timestep: int):
         self.timestep = timestep
-        v = self.verts_rest if self.pose_fn is None else self.pose_fn(self.verts_rest, timestep)
+        if self.flame is not None:
+            v = self.flame.mesh_at(self.flame_param, timestep)
+        else:
+            v = self.verts_rest if self.pose_fn is None else self.pose_fn(self.verts_rest, timestep)
         self.update_mesh_properties(v)
 
     # ---- getters: the reference route (eager) ----

@@ -191,3 +191,70 @@ def avatar_splats(P=100_000, n_faces=10_144, seed=0, sh_degree=3, scale_gain=1.0
     f_rest = 0.08 * torch.randn(P, M - 1, 3, generator=g)
     return dict(_xyz=xyz, _scaling=scaling, _rotation=rotation, _opacity=opacity, _features_dc=f_dc,
                 _features_rest=f_rest, binding=binding)
+
+
+def flame_like_model(seed: int = 0, n_shape: int = 300, n_expr: int = 100, n_lat: int = 52, n_lon: int = 98):
+    """A model with FLAME's array shapes and structure, in FlameHead's buffer layout (the licensed arrays are not part of
+    this project).  The template is `head_mesh(n_lat, n_lon)` (5000 vertices by default) plus 120 teeth-like vertices
+    in 8 rows of 15 that, as FlameHead.add_teeth builds them, have one-hot skinning weights (upper rows on the neck,
+    lower rows on the jaw), zero posedirs and J_regressor columns, zero expression directions and shape directions
+    copied from the nearest head vertex.  Shape / expression / pose directions are low-frequency in position (posed
+    meshes stay smooth), joint regressors are convex averages of nearby vertices, skinning weights are geometric and
+    sum to 1.  Joints: 0 global, 1 neck, 2 jaw, 3 / 4 eyes; parents [-1, 0, 1, 1, 1].  Everything is drawn from
+    np.random.RandomState(seed), whose stream numpy keeps fixed across versions.  Returns a dict of CPU tensors plus
+    n_shape / n_expr."""
+    rs = np.random.RandomState(seed)
+    head, faces = head_mesh(n_lat, n_lon)
+    head = head.numpy().astype(np.float64)
+    Vh = head.shape[0]
+    # teeth: rows in add_teeth's order (upper root, lower root, upper edge, lower edge, upper root back, upper edge
+    # back, lower root back, lower edge back)
+    x = np.linspace(-0.03, 0.03, 15)
+    row_yz = [(-0.045, 0.085), (-0.095, 0.082), (-0.062, 0.088), (-0.078, 0.084),
+              (-0.045, 0.075), (-0.062, 0.078), (-0.095, 0.072), (-0.078, 0.074)]
+    teeth = np.concatenate([np.stack([x, np.full(15, y), np.full(15, z)], 1) for y, z in row_yz])
+    upper = np.concatenate([np.arange(15 * r, 15 * r + 15) for r in (0, 2, 4, 5)])
+    lower = np.concatenate([np.arange(15 * r, 15 * r + 15) for r in (1, 3, 6, 7)])
+    v = np.concatenate([head, teeth])
+    V, NB = v.shape[0], n_shape + n_expr
+    tf = []
+    for r0, r1 in ((0, 2), (1, 3), (4, 5), (6, 7)):   # a strip of 28 triangles between two rows
+        for i in range(14):
+            a, b, c, d = 15 * r0 + i, 15 * r0 + i + 1, 15 * r1 + i, 15 * r1 + i + 1
+            tf += [(a, c, b), (b, c, d)]
+    faces = torch.cat([faces, torch.tensor(np.asarray(tf, np.int64) + Vh)])
+
+    def smooth(n_fields, amp):   # (V, 3, n_fields): a * sin(w . x + phi), |w| up to ~2 cycles per head
+        w = rs.normal(0.0, 12.0, size=(n_fields, 3))
+        phi = rs.uniform(0, 2 * np.pi, size=(n_fields, 3))
+        a = rs.normal(0.0, 1.0, size=(n_fields, 3)) * amp[:, None]
+        arg = head @ w.T                                   # (Vh, n_fields)
+        return a.T[None] * np.sin(arg[:, None, :] + phi.T[None])
+
+    decay = lambda n, s: s / (1.0 + np.arange(n) / 30.0)  # noqa: E731
+    sd = np.concatenate([smooth(n_shape, decay(n_shape, 2e-3)), smooth(n_expr, decay(n_expr, 1.5e-3))], axis=2)
+    nearest = np.argmin(((teeth[:, None, :] - head[None]) ** 2).sum(-1), axis=1)
+    sd_teeth = np.zeros((120, 3, NB))
+    sd_teeth[:, :, :n_shape] = sd[nearest, :, :n_shape]
+    shapedirs = np.concatenate([sd, sd_teeth])
+    pd = smooth(36, np.full(36, 4e-3))                     # (Vh, 3, 36)
+    posedirs = np.concatenate([pd, np.zeros((120, 3, 36))]).reshape(3 * V, 36).T.copy()
+    centres = np.array([[0.0, -0.02, 0.0], [0.0, -0.14, -0.01], [0.0, -0.07, 0.05],
+                        [0.035, 0.03, 0.09], [-0.035, 0.03, 0.09]])
+    J_regressor = np.zeros((5, V))
+    for j, c in enumerate(centres):
+        near = np.argsort(((head - c) ** 2).sum(-1))[:24]
+        wts = rs.uniform(0.5, 1.5, size=24)
+        J_regressor[j, near] = wts / wts.sum()
+    sig = np.array([0.25, 0.07, 0.05, 0.02, 0.02])
+    d2 = ((head[:, None, :] - centres[None]) ** 2).sum(-1)
+    w = np.exp(-d2 / sig ** 2) * np.array([0.2, 1.0, 1.0, 1.0, 1.0])
+    w = w / w.sum(1, keepdims=True)
+    wt = np.zeros((120, 5))
+    wt[upper, 1] = 1.0
+    wt[lower, 2] = 1.0
+    lbs_weights = np.concatenate([w, wt])
+    f32 = lambda a: torch.tensor(np.asarray(a, np.float32))  # noqa: E731
+    return dict(v_template=f32(v), shapedirs=f32(shapedirs), posedirs=f32(posedirs), J_regressor=f32(J_regressor),
+                parents=torch.tensor([-1, 0, 1, 1, 1], dtype=torch.int64), lbs_weights=f32(lbs_weights), faces=faces,
+                n_shape=n_shape, n_expr=n_expr)

@@ -266,6 +266,59 @@ int32_t gab200_face_frame_backward(int32_t F, int32_t V, const float* verts, con
                                    const float* dL_dface_center, const float* dL_dface_orien_mat,
                                    const float* dL_dface_scaling, float* dL_dverts, void* stream);
 
+/* FLAME head: blendshapes + linear blend skinning of one mesh per call, with its backward.  Replaces
+ * FlameHead.forward(shape, expr, rotation, neck, jaw, eyes, translation, zero_centered_at_root_node=False,
+ * return_landmarks=False, return_verts_cano=True, static_offset=...) and its autograd (flame_model/flame.py:485-558,
+ * flame_model/lbs.py:25-57,101-304).  The model arrays are inputs (FlameHead's buffers in its layout; NB =
+ * n_shape + n_expr); the caller precomputes J_template = J_regressor v_template and J_shapedirs = J_regressor shapedirs
+ * once per model.  Per-timestep parameters are (T, k) tables read at the device row index `row` (NULL = row 0), so a
+ * captured CUDA graph can replay any timestep; a row outside [0, T) turns every output of the call into NaN and the
+ * backward into a no-op.  Forward: 2 launches, backward: 2 launches, no host synchronisation. */
+typedef struct gab200_flame_args {
+  uint32_t abi_version;
+  int32_t V, n_shape, n_expr;
+  int32_t J;                    /* joints: must be 5 (global, neck, jaw, left eye, right eye) */
+  int32_t T;                    /* rows of the per-timestep tables */
+  /* model */
+  const float* v_template;      /* [V,3] */
+  const float* shapedirs;       /* [V,3,NB] */
+  const float* posedirs;        /* [(J-1)*9, V*3] */
+  const float* J_regressor;     /* [J,V] dense */
+  const float* lbs_weights;     /* [V,J] */
+  const int32_t* parents;       /* [J] device; parents[j] in [0, j) for j >= 1 (otherwise the outputs are NaN) */
+  const float* J_template;      /* [J,3] */
+  const float* J_shapedirs;     /* [J,3,NB] */
+  /* parameters */
+  const int32_t* row;           /* device, one int32, or NULL (= row 0) */
+  const float* shape;           /* [n_shape] or NULL (= 0) */
+  const float* expr;            /* [T,n_expr] */
+  const float* rotation;        /* [T,3] */
+  const float* neck;            /* [T,3] */
+  const float* jaw;             /* [T,3] */
+  const float* eyes;            /* [T,6] */
+  const float* translation;     /* [T,3] */
+  const float* static_offset;   /* [V,3] or NULL (= 0) */
+  /* outputs */
+  float* verts;                 /* [V,3] */
+  float* verts_cano;            /* [V,3] (v_shaped) or NULL */
+  void* workspace;              /* gab200_flame_workspace_bytes(V, n_shape, n_expr) bytes, 256-byte aligned: written by the
+                                   forward, read by the backward of the same call */
+  /* gradients (backward): ADDED into; NULL = not wanted.  The (T,k) ones are touched in row `row` only.  Without
+     grad_shape the shape columns of shapedirs (n_shape of NB) are not read. */
+  float* grad_shape;            /* [n_shape] */
+  float* grad_expr;             /* [T,n_expr] */
+  float* grad_rotation;         /* [T,3] */
+  float* grad_neck;             /* [T,3] */
+  float* grad_jaw;              /* [T,3] */
+  float* grad_eyes;             /* [T,6] */
+  float* grad_translation;      /* [T,3] */
+  float* grad_static_offset;    /* [V,3] */
+} gab200_flame_args;
+size_t gab200_flame_workspace_bytes(int32_t V, int32_t n_shape, int32_t n_expr);
+int32_t gab200_flame_forward(const gab200_flame_args* args, void* stream);
+/* dL_dverts [V,3]: gradient of the loss w.r.t. `verts` of the forward that filled args->workspace. */
+int32_t gab200_flame_backward(const gab200_flame_args* args, const float* dL_dverts, void* stream);
+
 /* Mean absolute error between a rendered image (n = 3*H*W floats) and a uint8 ground truth (value/255), with its
  * gradient, in one pass: *loss = mean |img - gt/255|, grad[i] = sign(img[i] - gt[i]/255) / n.  `loss` is zeroed by the
  * library.  Replaces `l1_loss(image, gt_image)` + its autograd and the float32 upload of the ground truth
